@@ -1,6 +1,6 @@
 """Benchmark of the multi_input_vocoder generator forward on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -20,6 +20,10 @@ device-resident loop run back to back for >= 3 s (clocks and power sampled), the
 figure compared with the sustained tensor peak.  `extra` = the other BASELINE
 configs through the public API: cfg3 (256 x 8 s split over the N ranks, strong
 scaling) and cfg5 (64 x 6 s split over the ranks, multi-input vs unit-only).
+
+--dump-outputs DIR writes the waveform the last timed step returned on rank 0, (16, 1, 64000) float32, as
+DIR/waveform.npy.  Inputs and weights are seeded, so two builds run with the same arguments can be compared
+output for output.
 """
 import argparse
 import json
@@ -32,6 +36,7 @@ import time
 import types
 import warnings
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -262,7 +267,12 @@ def main():
     ap.add_argument("--no-extra", action="store_true", help="skip the sustained loop and the cfg3 / cfg5 extras")
     ap.add_argument("--knob", action="append", default=[], help="debug knob k=v passed to l2s_debug_set")
     ap.add_argument("--layers", action="store_true", help="also print a per-launch time table to stderr")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the waveform of the last timed step to DIR/waveform.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     args.warmup = max(args.warmup, 3)
 
     rank = int(os.environ.get("RANK", "0"))
@@ -331,6 +341,9 @@ def main():
     ev1.record()
     sync_all()
     ms = ev0.elapsed_time(ev1)
+    if args.dump_outputs and rank == 0:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "waveform.npy"), y.cpu().numpy())
     # host time to ISSUE one step (no synchronisation): if it approaches ms_per_step the path is launch bound
     t_h0 = time.perf_counter()
     for _ in range(args.steps):

@@ -1,4 +1,4 @@
-"""The vocoder service's call sequence, restated for the GPU box (where /root/reference does not exist).
+"""The vocoder service's call sequence, restated so that it runs without the upstream repository.
 
 Follows multi_input_vocoder/inference_server.py: module imports (:28), init() (:85-130: JSON -> AttrDict h,
 h.code_dict_path, h.text_supervision from the environment, MelCodeGenerator(h).to(device),

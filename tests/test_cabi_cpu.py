@@ -7,6 +7,7 @@ import re
 
 import pytest
 import torch
+import torch.multiprocessing as mp
 
 from oracle import vocoder_oracle as vo
 
@@ -79,22 +80,41 @@ def test_create_validates_without_cuda(pkg):
     lib.l2s_destroy(hnd)
 
 
-@pytest.mark.skipif(torch.cuda.is_available(), reason="checks the no-GPU failure mode")
-def test_finalize_fails_loudly_without_a_gpu(pkg):
+def _finalize_without_a_gpu(q):
+    import sys
+    sys.path.insert(0, ROOT)
+    import __graft_entry__ as ge
+    pkg = ge.load_package()
     lib = pkg._cabi.load()
-    h = vo.shipped_config()
-    g = pkg.MelCodeGenerator(pkg.AttrDict(h))
+    g = pkg.MelCodeGenerator(pkg.AttrDict(vo.shipped_config()))
     cfg = g._config()
     hnd = C.c_void_p()
-    assert lib.l2s_create(C.byref(cfg), C.byref(hnd)) == 0
-    keep = []
+    created = lib.l2s_create(C.byref(cfg), C.byref(hnd))
+    keep, rejected = [], []
     for name, t in g._plain_weights().items():
         t = t.float().contiguous()
         keep.append(t)
-        assert lib.l2s_set_weight(hnd, name.encode(), t.data_ptr(), t.numel()) == 0, name
-    assert lib.l2s_finalize(hnd, 0) == pkg._cabi.ERR_CUDA
-    assert b"no CPU fallback" in lib.l2s_last_error(hnd)
+        if lib.l2s_set_weight(hnd, name.encode(), t.data_ptr(), t.numel()) != 0:
+            rejected.append(name)
+    q.put((created, rejected, lib.l2s_finalize(hnd, 0), lib.l2s_last_error(hnd)))
     lib.l2s_destroy(hnd)
+
+
+def test_finalize_fails_loudly_without_a_gpu(pkg, monkeypatch):
+    """The library in a process that sees no CUDA device (CUDA_VISIBLE_DEVICES empty), so this also runs on a GPU
+    machine."""
+    monkeypatch.setenv("CUDA_VISIBLE_DEVICES", "")
+    ctx = mp.get_context("spawn")
+    q = ctx.Queue()
+    p = ctx.Process(target=_finalize_without_a_gpu, args=(q,))
+    p.start()
+    created, rejected, status, err = q.get(timeout=300)
+    p.join(timeout=60)
+    assert p.exitcode == 0
+    assert created == pkg._cabi.OK
+    assert rejected == []
+    assert status == pkg._cabi.ERR_CUDA
+    assert b"no CPU fallback" in err
 
 
 def test_host_class_surface(pkg):

@@ -1,8 +1,8 @@
 """The drop-in boundary as the reference's own scripts reach it: `from models_multi_input import MelCodeGenerator`
 (multi_input_vocoder/inference.py:28, inference_server.py:28).  CPU side: import resolution, the launcher's
-precedence over the script-directory sibling, and -- where /root/reference exists (the build container) -- the
-UNMODIFIED reference inference.py executed through the launcher up to the generator call, which on a machine
-without a B200 must fail loudly (there is no CPU fallback)."""
+precedence over the script-directory sibling, and -- when L2S_REFERENCE_DIR names a checkout of the upstream
+lip2speech-unit repository -- the UNMODIFIED reference inference.py executed through the launcher up to the generator
+call, which on a machine without a B200 must fail loudly (there is no CPU fallback)."""
 import json
 import os
 import shutil
@@ -19,8 +19,8 @@ PKG_DIR = os.path.join(ROOT, "lip2speech-unit_b200")
 LAUNCHER = os.path.join(PKG_DIR, "dropin.py")
 CALLER = os.path.join(ROOT, "tests", "dropin_caller", "inference_like.py")
 STUBS = os.path.join(ROOT, "tests", "stubs")
-REF = "/root/reference"
-REF_SCRIPT = os.path.join(REF, "multi_input_vocoder", "inference.py")
+REF = os.path.abspath(os.environ["L2S_REFERENCE_DIR"]) if os.environ.get("L2S_REFERENCE_DIR") else None   # upstream checkout
+REF_SCRIPT = os.path.join(REF, "multi_input_vocoder", "inference.py") if REF else None
 
 
 def _run(cmd, env_extra=None, cwd=None):
@@ -78,7 +78,7 @@ def make_job(tmp, root, precision=None):
     return cfg_path, ckpt, os.path.join(tmp, "label", "test.tsv"), os.path.join(tmp, "label", "dict.unt.txt"), sd, h
 
 
-@pytest.mark.skipif(not os.path.isfile(REF_SCRIPT), reason="the reference tree only exists in the build container")
+@pytest.mark.skipif(not (REF_SCRIPT and os.path.isfile(REF_SCRIPT)), reason="set L2S_REFERENCE_DIR to an upstream lip2speech-unit checkout")
 def test_unmodified_reference_inference_py_through_the_launcher(pkg, tmp_path):
     """`python dropin.py <reference>/multi_input_vocoder/inference.py cfg manifest dict --checkpoint_file ... --debug`:
     the reference's argument parsing, parse_manifest, MelCodeDataset, init_worker (MelCodeGenerator(h).to(device),

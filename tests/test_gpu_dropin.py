@@ -2,9 +2,9 @@
 (multi_input_vocoder/inference_server.py:85-146): a separate process runs `dropin.py <caller script>`, the caller does
 `from models_multi_input import MelCodeGenerator` next to a sibling of that name, builds the generator from the JSON
 config, loads a weight-normed checkpoint, vocodes the shipped lrs3 sample rows one at a time and writes int16 wav
-files; they are compared with the oracle.  (/root/reference does not exist on the GPU box, so the caller is the
+files; they are compared with the oracle.  (The upstream repository is not part of this one, so the caller is the
 restated tests/dropin_caller/inference_like.py; the unmodified reference script is run through the same launcher
-by tests/test_dropin_cpu.py in the build container.)"""
+by tests/test_dropin_cpu.py when L2S_REFERENCE_DIR names an upstream checkout.)"""
 import os
 import sys
 
