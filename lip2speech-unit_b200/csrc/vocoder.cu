@@ -278,6 +278,15 @@ int build_layers(l2s_vocoder* v) {
     v->rb_c2.push_back(s2);
   }
   if (ch > 64) return fail(v, L2S_ERR_UNSUPPORTED, "final channel count must be <= 64");
+  // Every conv reads its input rows with pitch cin_pad, but the epilogues write activations with pitch cout and the
+  // workspace holds len * ch elements per stage.  Only the front end writes conv_pre's input with the padded pitch, so
+  // any other layer whose input channels get padded (C > 64 and not a multiple of 64) would read misaligned rows.
+  for (const ConvLayer& L : v->convs) {
+    if (&L == &v->convs[v->conv_pre] || L.cin_pad == L.cin) continue;
+    char b[160];
+    snprintf(b, sizeof b, "%s has %d input channels: channel counts above 64 must be multiples of 64", L.name.c_str(), L.cin);
+    return fail(v, L2S_ERR_UNSUPPORTED, b);
+  }
   v->expected["conv_post.weight"] = (long long)ch * 7;
   v->expected["conv_post.bias"] = 1;
   v->expected["dict.weight"] = (long long)c.num_embeddings * E;
@@ -1085,7 +1094,18 @@ int forward_impl(l2s_vocoder* v, void* stream, const int64_t* code, const void* 
   else if (pp.c == 32 && g_knobs.post_rows) post_rows_kernel<32><<<grid_rows, kPostTile, 0, st>>>(pp);
   else if (pp.c == 16) post_kernel<16><<<grid, kPostTile, (kPostTile + 6) * post_pitch(pp.c) * sizeof(float), st>>>(pp);
   else if (pp.c == 32) post_kernel<32><<<grid, kPostTile, (kPostTile + 6) * post_pitch(pp.c) * sizeof(float), st>>>(pp);
-  else post_kernel<0><<<grid, kPostTile, (kPostTile + 6) * post_pitch(pp.c) * sizeof(float), st>>>(pp);
+  else {
+    // C = 48 / 64: the staged tile ((kPostTile + 6) rows of C + 4 floats, 71 KB at C = 64) is larger than the 48 KB of
+    // dynamic shared memory a launch gets without opting in
+    static bool configured[64] = {false};
+    if (v->device >= 0 && v->device < 64 && !configured[v->device]) {
+      if ((e = cudaFuncSetAttribute(post_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                    (int)((kPostTile + 6) * post_pitch(kPostMaxC) * sizeof(float)))) != cudaSuccess)
+        return fail(v, L2S_ERR_CUDA, std::string("post: ") + cudaGetErrorString(e));
+      configured[v->device] = true;
+    }
+    post_kernel<0><<<grid, kPostTile, (kPostTile + 6) * post_pitch(pp.c) * sizeof(float), st>>>(pp);
+  }
   timed_end(v, st);
   if ((e = cudaGetLastError()) != cudaSuccess) return fail(v, L2S_ERR_CUDA, std::string("post: ") + cudaGetErrorString(e));
   return L2S_OK;
